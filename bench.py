@@ -1,6 +1,10 @@
-"""bench.py — driver contract (see task statement): one JSON line per run.
+"""bench.py — benchmark of the flagship workload: one JSON line per run.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload e2e|align] [--impl ours|reference]
+                    [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the timed path computed in its last step as DIR/<name>.npy (float32 / float64, at
+most 64 MB in all); the inputs are seeded, so two builds run with the same arguments can be compared array by array.
 
 Workloads
   e2e   : (default) BASELINE.json metric — audio-seconds/second of whisper_timestamped.transcribe() for
@@ -140,7 +144,40 @@ def dtw_kernel_name(nseg, T):
     return "dtw_small_kernel<32,1>" if T <= 31 else "dtw_warp_kernel<float>"
 
 
-def run_align(args, rank, world):
+DUMP_LIMIT = 64 << 20
+COST_SAMPLE = 1 << 20
+
+
+def write_outputs(dirname, arrays):
+    """Each array as DIR/<name>.npy; float32 / float64 only, at most DUMP_LIMIT bytes in all."""
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT, f"outputs of {total} bytes exceed the {DUMP_LIMIT}-byte dump limit"
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
+def transcribe_arrays(res):
+    """The result dict of transcribe() as flat float64 arrays: every numeric segment and word field, the tokens of all
+    segments back to back, per-segment token and word counts, and the UTF-8 bytes of the text and of the word texts."""
+    def numeric(v):
+        return isinstance(v, (int, float)) and not isinstance(v, bool)
+
+    segs = res["segments"]
+    words = [w for s in segs for w in s.get("words", [])]
+    out = {"text_utf8": np.frombuffer(res["text"].encode(), dtype=np.uint8).astype(np.float64),
+           "tokens": np.array([t for s in segs for t in s["tokens"]], dtype=np.float64),
+           "tokens_per_segment": np.array([len(s["tokens"]) for s in segs], dtype=np.float64),
+           "words_per_segment": np.array([len(s.get("words", [])) for s in segs], dtype=np.float64),
+           "word_text_utf8": np.frombuffer("\n".join(w["text"] for w in words).encode(), dtype=np.uint8).astype(np.float64)}
+    for prefix, items in (("segment_", segs), ("word_", words)):
+        for k in sorted({k for x in items for k, v in x.items() if numeric(v)}):
+            out[prefix + k] = np.array([x.get(k, np.nan) for x in items], dtype=np.float64)
+    return out
+
+
+def run_align(args, rank, world, keep_outputs=False):
     import torch
     from whisper_timestamped.alignment import plan_segments, attn_prep, dtw, dtw_descriptors, _segs_to_device
     dev = torch.device("cuda", int(os.environ.get("LOCAL_RANK", 0)))
@@ -189,6 +226,14 @@ def run_align(args, rank, world):
     wall = time.perf_counter() - t0
     total_ms = e0.elapsed_time(e1)
     clocks = sampler.stop() if rank == 0 else None
+    outputs = None
+    if keep_outputs:
+        # the last timed step's buffers, copied before the host-buffer passes below reuse `cost`
+        n = min(COST_SAMPLE, plan.cost_elems)
+        idx = np.sort(np.random.default_rng(0).choice(plan.cost_elems, size=n, replace=False))
+        outputs = {"jumps": out["jumps"].cpu().numpy().astype(np.float64),
+                   "cost_sample": cost[torch.from_numpy(idx).to(dev)].cpu().numpy(),
+                   "cost_sample_index": idx.astype(np.float64)}
     # host-buffer e2e: qk slices are device-resident products of the decoder in the real pipeline, so the
     # host-facing e2e of this micro-workload = descriptors H2D + jumps D2H each step
     e2e_t = []
@@ -212,6 +257,7 @@ def run_align(args, rank, world):
         "e2e_segments_per_s": nseg / float(np.median(e2e_t)),
         "h2d": int(plan.segs.nbytes), "d2h": int(plan.jumps_elems * 4),
         "peaks": peaks, "alg_bytes": alg, "jumps_checksum": int(out["jumps"].sum().item()),
+        "outputs": outputs,
     }
     return res
 
@@ -368,6 +414,7 @@ def run_e2e(args, rank, world, local):
     barrier()
     wall = time.perf_counter() - t0
     ms = e0.elapsed_time(e1)
+    timed_res = res
     stages = eng.stage_ms()
     eng.profile = False
     if rank == 0 and os.environ.get("WTS_BENCH_VERBOSE"):
@@ -397,7 +444,7 @@ def run_e2e(args, rank, world, local):
            "clocks": clocks, "launches": launches, "segments": len(res["segments"]), "tokens": ntok, "words": nw,
            "h2d": int(mine.nbytes), "d2h": int(len(json.dumps(res["segments"]))) if rank == 0 else 0, "wall_s": wall,
            "decode_steps": getattr(eng, "decode_steps_run", 0), "small_batch_steps": eng.small_batch_steps,
-           "result": res if rank == 0 else None}
+           "result": res if rank == 0 else None, "timed_result": timed_res if rank == 0 else None}
     if rank == 0 and not args.no_roofline:
         peaks = measured_peaks()
         out["roofline"] = gemm_roofline(eng, peaks)
@@ -572,7 +619,13 @@ def main():
     ap.add_argument("--recipe", default="default", choices=sorted(RECIPES))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-roofline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3)
     SYNTH_KW.clear()
     SYNTH_KW.update(RECIPES[args.recipe])
@@ -621,6 +674,8 @@ def main():
 
     if args.workload == "e2e":
         res = run_e2e(args, rank, world, local)
+        if rank == 0 and args.dump_outputs:
+            write_outputs(args.dump_outputs, transcribe_arrays(res["timed_result"]))
         if rank == 0:
             line = {
                 "metric": metric_name,
@@ -661,7 +716,9 @@ def main():
                 line["cpu_baseline"] = cb
             print(json.dumps(line))
     else:
-        res = run_align(args, rank, world)
+        res = run_align(args, rank, world, keep_outputs=bool(args.dump_outputs) and rank == 0)
+        if res["outputs"] is not None:
+            write_outputs(args.dump_outputs, res["outputs"])
         vals = [res["segments_per_s"]]
         ms = [res["ms_total"]]
         if world > 1:
